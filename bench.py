@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the headline measurement (BASELINE.json metric) for the filterpy hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one fused predict+update of a 2^20-filter bank, dim_x=4, dim_z=2, fp32, every
 filter with its own F/H/Q/R (BASELINE.json configs[1]).  Weak scaling: every rank owns its own
@@ -33,6 +33,7 @@ N_FILTERS = 1 << 20
 DIM_X, DIM_Z = 4, 2
 BYTES_PER_FILTER_STEP = (2 * DIM_X + 4 * DIM_X * DIM_X + DIM_Z + DIM_Z * DIM_X + DIM_Z * DIM_Z) * 4  # 344
 Z_RING = 4
+DUMP_FILTERS = 1 << 19       # --dump-outputs: filters sampled from the bank (x and P of all 2^20 would be 80 MB)
 METRIC = "kf_predict_update_filter_steps_per_sec"
 UNIT = "filter-steps/s"
 WORKLOAD = "kf_bank 2^20 filters dim_x=4 dim_z=2 fp32, per-filter F/H/Q/R, fused predict+update"
@@ -163,13 +164,10 @@ class ClockSampler:
 
 # ----------------------------------------------------------------------------- CPU legs
 def reference_importable():
-    """The unmodified reference (filterpy 1.4.5) when a copy is importable on this box: baseline/_ref
-    (pip --target install made by __graft_entry__.build() where /root/reference exists) or
-    /root/reference itself.  Returns the sys.path entry or None."""
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(cand, "filterpy", "kalman")):
-            return cand
-    return None
+    """The unmodified reference (filterpy 1.4.5) when __graft_entry__.build() installed a copy under
+    oracle/_ref (oracle/reference.py).  Returns the sys.path entry or None."""
+    from oracle import reference
+    return reference.importable()
 
 
 def _loop_port_worker(args):
@@ -328,7 +326,9 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize(dev)
 
     def reset():
-        kf.x = x0; kf.P = P0
+        # in place: the captured graph and the cached launch arguments hold the addresses of x and P,
+        # so every timed step, replayed or direct, advances the state a caller reads
+        kf.x.copy_(x0); kf.P.copy_(P0)
 
     def max_over_ranks(ms):
         if world > 1:
@@ -373,6 +373,11 @@ def run_ours(args, rank, world, local_rank):
     per_launch_ms = np.array([evs[r].elapsed_time(evs[r + 1]) / Z_RING for r in range(reps)] +
                              [evs[reps + i].elapsed_time(evs[reps + i + 1]) for i in range(rem)])
     value = world * N * K / (total_ms * 1e-3)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # the posterior of the last timed step, for a fixed sample of the filters
+        sel = torch.from_numpy(np.sort(np.random.default_rng(0).choice(N, DUMP_FILTERS, replace=False))).to(dev)
+        dump = {"x": kf.x.index_select(0, sel).cpu().numpy(), "P": kf.P.index_select(0, sel).cpu().numpy()}
 
     # ---- e2e: host buffers, copies inside the timed region -----------------------------------
     # Every step copies that step's measurements from pinned host memory to the device
@@ -484,6 +489,10 @@ def run_ours(args, rank, world, local_rank):
             "c_port": {"value": cp, "cores": cores, "sample": "2^19 filters x 4 steps fp64, %.1f s" % cp_wall},
         }
     print(json.dumps(line), flush=True)
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
 
 
 def timed_steps(fn, reps, warm, dev, max_over_ranks, barrier):
@@ -710,7 +719,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch every step directly instead of CUDA-graph replays")
     ap.add_argument("--no-pin", action="store_true", help="do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--no-extra", action="store_true", help="skip the C2-diagnostics / C3 / C4 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the posterior of the last one as DIR/x.npy (N,4) and "
+                         "DIR/P.npy (N,4,4), fp32, for a fixed seeded sample of 2^19 of rank 0's filters")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

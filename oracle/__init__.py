@@ -13,9 +13,8 @@ It is the *checker* for the CUDA path, never the product: only ``tests/``,
 imports it and the product path has no CPU fallback.
 
 Parity pinning: the oracle is pinned against outputs of the unmodified
-reference (rlabbe/filterpy 1.4.5 @ 3b51149) imported in the build container;
-the generating script is ``tests/golden/make_golden.py`` and the vectors are
-committed under ``tests/golden/*.npz``.  ``tests/test_oracle_golden.py`` checks
-every oracle function against them (and, when ``/root/reference`` is present,
-against the live reference too).
+reference (rlabbe/filterpy 1.4.5 @ 3b51149); the generating script is
+``tests/golden/make_golden.py`` and the vectors are committed under
+``tests/golden/*.npz``.  ``tests/test_oracle_golden.py`` checks every oracle
+function against them.
 """

@@ -1,14 +1,14 @@
 #!/usr/bin/env python
 """Generate the golden vectors under tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists):
+Run with FILTERPY_REFERENCE naming a source checkout of the reference:
 
-    python tests/golden/make_golden.py
+    FILTERPY_REFERENCE=<checkout> python tests/golden/make_golden.py
 
-It imports rlabbe/filterpy 1.4.5 (@ 3b51149) from /root/reference, feeds it the seeded
+It imports rlabbe/filterpy 1.4.5 (@ 3b51149) from that checkout, feeds it the seeded
 synthetic inputs of ``filterpy_b200.common.workloads`` and stores inputs + the reference's
-outputs as small ``.npz`` files.  The reference cannot travel to the GPU box, the vectors
-can: tests compare the oracle (``oracle/``) and the CUDA path against them.
+outputs as small ``.npz`` files.  The tests need only the vectors, not the reference:
+they compare the oracle (``oracle/``) and the CUDA path against them.
 """
 import os
 import sys
@@ -18,7 +18,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["FILTERPY_REFERENCE"])
 
 from filterpy.kalman import KalmanFilter, UnscentedKalmanFilter, MerweScaledSigmaPoints  # noqa: E402
 from filterpy.kalman import predict as kf_predict_proc, update as kf_update_proc          # noqa: E402
@@ -454,6 +454,49 @@ def gen_mm():
     save("mm", **out)
 
 
+# ----------------------------------------------------------------------------- spot checks
+def gen_spot_checks():
+    """The reference's public functions called the way a user calls them (seeded global RNG):
+    systematic / residual / multinomial resample, a 5-filter KF bank and the RTS smoother of C1."""
+    out = {}
+    w = wl.resample_weights(20000, "heavy", seed=5)
+    np.random.seed(123); st = np.random.get_state()
+    out["sys_idx"] = systematic_resample(w)
+    np.random.set_state(st)
+    out.update(sys_w=w, sys_u=np.random.random())
+    b = wl.kf_bank_cv2d(5, seed=11, steps=2)
+    xs, Ps = [], []
+    for f in range(5):
+        kf = KalmanFilter(4, 2); kf.x = b["x"][f].copy(); kf.P = b["P"][f].copy()
+        kf.F, kf.H, kf.Q, kf.R = b["F"][f], b["H"][f], b["Q"][f], b["R"][f]
+        for t in range(2):
+            kf.predict(); kf.update(b["zs"][t, f])
+        xs.append(kf.x); Ps.append(kf.P)
+    out.update({"kf_" + k: v for k, v in b.items()})
+    out.update(kf_ref_x=np.array(xs), kf_ref_P=np.array(Ps))
+    rng = np.random.default_rng(5)
+    for N in [3, 50, 3001]:
+        w = rng.random(N) ** 3
+        w /= w.sum()
+        np.random.seed(21); idx = residual_resample(w.copy())
+        k = int(np.floor(N * w).astype(int).sum())
+        np.random.seed(21)
+        out.update({"res%d_w" % N: w, "res%d_U" % N: np.random.random(N - k), "res%d_idx" % N: idx})
+    rng = np.random.default_rng(0)
+    w = rng.random(5000) ** 3
+    w /= w.sum()
+    np.random.seed(9); idx = multinomial_resample(w)
+    np.random.seed(9)
+    out.update(mn_w=w, mn_U=np.random.random(len(w)), mn_idx=idx)
+    c = wl.kf_single_cv2d(T=50, seed=2)
+    kf = KalmanFilter(4, 2)
+    kf.x = c["x"].copy(); kf.P = c["P"].copy(); kf.F, kf.H, kf.Q, kf.R = c["F"], c["H"], c["Q"], c["R"]
+    mu, cov, _, _ = kf.batch_filter(list(c["zs"]))
+    x, P, K, Pp = kf.rts_smoother(mu, cov)
+    out.update(rts_F=c["F"], rts_Q=c["Q"], rts_mu=mu, rts_cov=cov, rts_x=x, rts_P=P, rts_K=K, rts_Pp=Pp)
+    save("spot_checks", **out)
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1:                       # e.g. `make_golden.py gen_ukf_julier`: only the named generators
         for g in sys.argv[1:]:
@@ -470,3 +513,4 @@ if __name__ == "__main__":
     gen_mm()
     gen_ukf_julier()
     gen_ukf_user()
+    gen_spot_checks()

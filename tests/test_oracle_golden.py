@@ -1,14 +1,9 @@
 """The oracle (oracle/) against the golden vectors produced by the unmodified reference
-(tests/golden/make_golden.py) — and against the live reference when /root/reference exists."""
-import os
-import sys
-
+(tests/golden/make_golden.py)."""
 import numpy as np
 import pytest
 
 from oracle import kf as okf, ukf as oukf, resample as ors
-
-HAVE_REF = os.path.isdir("/root/reference/filterpy")
 
 
 def close(a, b, rtol=1e-9, atol=1e-11):
@@ -188,28 +183,18 @@ def test_resample_golden(golden):
                     fn(w, U)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference not present (GPU box)")
-def test_live_reference_resample_and_kf():
-    sys.path.insert(0, "/root/reference")
-    from filterpy.monte_carlo import systematic_resample
-    from filterpy.kalman import KalmanFilter
-    from filterpy_b200.common import workloads as wl
-    w = wl.resample_weights(20000, "heavy", seed=5)
-    np.random.seed(123); st = np.random.get_state()
-    ref = systematic_resample(w)
-    np.random.set_state(st); u = np.random.random()
+def test_live_reference_resample_and_kf(golden):
+    """systematic_resample(w) after np.random.seed(123), and five reference KalmanFilter objects over
+    two steps (tests/golden/make_golden.py:gen_spot_checks)."""
+    g = golden("spot_checks")
+    w, u, ref = g["sys_w"], float(g["sys_u"]), g["sys_idx"]
     assert np.array_equal(ors.systematic_resample_vec(w, u), ref)
     assert np.array_equal(ors.systematic_resample_c(w, u), ref)
-    b = wl.kf_bank_cv2d(5, seed=11, steps=2)
-    o = None; x, P = b["x"], b["P"]
+    o = None; x, P = g["kf_x"], g["kf_P"]
     for t in range(2):
-        o = okf.kf_step_bank(x, P, b["zs"][t], b["F"], b["H"], b["Q"], b["R"]); x, P = o["x"], o["P"]
+        o = okf.kf_step_bank(x, P, g["kf_zs"][t], g["kf_F"], g["kf_H"], g["kf_Q"], g["kf_R"]); x, P = o["x"], o["P"]
     for f in range(5):
-        kf = KalmanFilter(4, 2); kf.x = b["x"][f].copy(); kf.P = b["P"][f].copy()
-        kf.F, kf.H, kf.Q, kf.R = b["F"][f], b["H"][f], b["Q"][f], b["R"][f]
-        for t in range(2):
-            kf.predict(); kf.update(b["zs"][t, f])
-        close(x[f], kf.x, 1e-12); close(P[f], kf.P, 1e-12)
+        close(x[f], g["kf_ref_x"][f], 1e-12); close(P[f], g["kf_ref_P"][f], 1e-12)
 
 
 # ------------------------------------------------------------------ §8f rows: multinomial resample, RTS smoother
@@ -246,20 +231,13 @@ def test_residual_oracle_vs_reference_vectors(golden):
     assert nonmono >= 10 and dep >= 1
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
-def test_residual_live_reference():
-    sys.path.insert(0, "/root/reference")
-    try:
-        from filterpy.monte_carlo import residual_resample
-    finally:
-        sys.path.remove("/root/reference")
-    rng = np.random.default_rng(5)
+def test_residual_live_reference(golden):
+    """residual_resample(w) after np.random.seed(21) (tests/golden/make_golden.py:gen_spot_checks)."""
+    g = golden("spot_checks")
     for N in [3, 50, 3001]:
-        w = rng.random(N) ** 3
-        w /= w.sum()
-        np.random.seed(21); ref = residual_resample(w.copy())
+        w, U, ref = g["res%d_w" % N], g["res%d_U" % N], g["res%d_idx" % N]
         k = int(np.floor(N * w).astype(int).sum())
-        np.random.seed(21); U = np.random.random(N - k)
+        assert len(U) == N - k
         assert np.array_equal(ors.residual_resample_vec(w, U), ref)
 
 
@@ -279,29 +257,15 @@ def test_rts_oracle_vs_reference_vectors(golden):
             close(got, g[name + "_" + key], rtol=1e-12, atol=1e-13)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
-def test_multinomial_and_rts_live_reference():
-    sys.path.insert(0, "/root/reference")
-    try:
-        from filterpy.monte_carlo import multinomial_resample
-        from filterpy.kalman import KalmanFilter
-    finally:
-        sys.path.remove("/root/reference")
-    rng = np.random.default_rng(0)
-    w = rng.random(5000) ** 3
-    w /= w.sum()
-    np.random.seed(9); ref = multinomial_resample(w)
-    np.random.seed(9); U = np.random.random(len(w))
+def test_multinomial_and_rts_live_reference(golden):
+    """multinomial_resample(w) after np.random.seed(9), and KalmanFilter.rts_smoother on the reference's
+    own batch_filter output of a 50-step C1 track (tests/golden/make_golden.py:gen_spot_checks)."""
+    g = golden("spot_checks")
+    w, U, ref = g["mn_w"], g["mn_U"], g["mn_idx"]
     assert np.array_equal(ors.multinomial_resample_c(w, U), ref)
-    from filterpy_b200.common import workloads as wl
-    c = wl.kf_single_cv2d(T=50, seed=2)
-    kf = KalmanFilter(4, 2)
-    kf.x = c["x"].copy(); kf.P = c["P"].copy(); kf.F, kf.H, kf.Q, kf.R = c["F"], c["H"], c["Q"], c["R"]
-    mu, cov, _, _ = kf.batch_filter(list(c["zs"]))
-    ref = kf.rts_smoother(mu, cov)
-    out = okf.rts_smoother(mu, cov, [c["F"]] * 50, [c["Q"]] * 50)
-    for a, b in zip(out, ref):
-        close(a, b, rtol=1e-12, atol=1e-13)
+    out = okf.rts_smoother(g["rts_mu"], g["rts_cov"], [g["rts_F"]] * 50, [g["rts_Q"]] * 50)
+    for a, key in zip(out, ["x", "P", "K", "Pp"]):
+        close(a, g["rts_" + key], rtol=1e-12, atol=1e-13)
 
 
 @pytest.mark.parametrize("nm", [2, 3])
